@@ -2,6 +2,7 @@
 """bench.py — agent-steps/s of the th_rl training hot path on N B200s (BASELINE.json metric).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload c2|c4|c5] [--no-extras]
+                    [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P \
         bench.py --gpus N --steps K --warmup W
 
@@ -20,6 +21,10 @@ workloads = the same measurement (value, e2e, roofline, clocks) for the other tw
          th_rl.trainer.train_one in one process per host core on a bounded sample of the same workload; when the staged
          reference is missing, the oracle port (oracle/thrl_oracle.c, all host threads).  The port's rate is reported next
          to it either way (`cpu_port`): it is ~10^3 x faster per core than the Python loop and the more conservative baseline.
+--dump-outputs DIR: after the timed steps of the headline workload, what its last step left a caller is written to
+         DIR/<name>.npy (see dump_outputs), so that two builds run with the same arguments can be compared output for output.
+
+bench.py writes nothing into the tree it runs from (which may be read-only): no bytecode caches either.
 """
 import argparse
 import json
@@ -34,6 +39,7 @@ ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
 
 MAX_STEPS = 100
+DUMP_BYTES = 50_000_000  # --dump-outputs writes about this much at most (plus the .npy headers)
 
 
 def _qcfg(n, states, actions, lo, hi, epochs, noise_prob=0):
@@ -289,7 +295,47 @@ def run_reference(args):
 
 
 # ------------------------------------------------------------------------------------------------------------ GPU legs
-def measure(name, wl, R, E, steps, warmup, e2e_chunks, ctx):
+def _sample(n, k):
+    """A fixed (seeded) sorted sample of k of range(n); all of it when k >= n."""
+    import numpy as np
+    return np.arange(n) if k >= n else np.sort(np.random.default_rng(0).choice(n, k, replace=False))
+
+
+def dump_outputs(batch, out, dump_dir):
+    """Writes what the last scan left its caller, as float32 / float64 .npy files in dump_dir:
+    stats.npy        [E, n, 4] f64: per epoch and agent, the sums over the runs of the epoch's mean reward, its square, the mean
+                     scaled action and its square (the kernel's fixed-point int64 sums over abi.THRL_STATS_SCALE_*);
+    and, for a fixed seeded sample of the runs (this rank's runs when there are several), the state the scan advanced in place:
+    q_agent<i>.npy   [S, states+1, actions] table of QTable agent i (the batch's table dtype);
+    counter_agent<i>.npy [S, states+1, actions] f64 visit counts of QTable agent i;
+    eps.npy [S, n] f64, price.npy [S] f64, mlp.npy [S, mlp_stride] f32 (parameters, Adam state and buffers of the MLP agents).
+    A stats array larger than a quarter of DUMP_BYTES keeps a fixed sample of its epochs; the runs fill the rest."""
+    import numpy as np
+    import torch
+    from th_rl_b200 import abi
+    os.makedirs(dump_dir, exist_ok=True)
+    g, R = batch.game, batch.n_runs
+    st = out.stats.cpu().numpy()
+    st = st[_sample(st.shape[0], max(1, (DUMP_BYTES // 4) // (st[0].size * 8)))]
+    scale = np.array([abi.THRL_STATS_SCALE_SUM, abi.THRL_STATS_SCALE_SQ] * 2)
+    np.save(os.path.join(dump_dir, "stats.npy"), st.astype(np.float64) / scale)
+    agents = [g.agent[i] for i in range(g.n_agents)]
+    cells = sum((s.states + 1) * s.actions for s in agents if s.kind == abi.THRL_AGENT_QTABLE)
+    per_run = cells * (batch.q.element_size() + 8) + g.mlp_stride * 4 + (g.n_agents + 1) * 8
+    runs = torch.as_tensor(_sample(R, max(1, (DUMP_BYTES - st.nbytes) // per_run)), device=batch.device)
+    q, counter = batch.q.index_select(0, runs), batch.counter.index_select(0, runs)
+    arrays = {"eps": batch.eps.index_select(0, runs), "price": batch.price.index_select(0, runs)}
+    for i, s in enumerate(agents):
+        if s.kind == abi.THRL_AGENT_QTABLE:
+            arrays["q_agent%d" % i] = abi.table_view(q, s)
+            arrays["counter_agent%d" % i] = abi.table_view(counter, s).cpu().numpy().view(np.uint32).astype(np.float64)
+    if batch.mlp is not None:
+        arrays["mlp"] = batch.mlp.index_select(0, runs)
+    for k, a in arrays.items():
+        np.save(os.path.join(dump_dir, k + ".npy"), a.cpu().numpy() if torch.is_tensor(a) else a)
+
+
+def measure(name, wl, R, E, steps, warmup, e2e_chunks, ctx, dump_dir=None):
     """value / e2e / roofline / clocks of one workload on this rank's GPU; collective maxima over ranks.  Returns a dict on
     every rank (rank 0 prints it)."""
     torch, np, dist, engine, _lib = ctx["torch"], ctx["np"], ctx["dist"], ctx["engine"], ctx["_lib"]
@@ -336,6 +382,8 @@ def measure(name, wl, R, E, steps, warmup, e2e_chunks, ctx):
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
     total_ms, kern_ms = t.tolist()
     value = agent_steps_rank * world * steps / (total_ms * 1e-3)
+    if dump_dir is not None and rank == 0:
+        dump_outputs(batch, out, dump_dir)
     del batch, out
     torch.cuda.empty_cache()
 
@@ -519,7 +567,8 @@ def run_ours(args):
         dist.init_process_group("nccl", device_id=dev)
     ctx = dict(torch=torch, np=np, dist=dist, engine=engine, _lib=_lib, world=world, rank=rank, dev=dev)
     wl = WORKLOADS[args.workload]
-    res = measure(args.workload, wl, args.runs_per_gpu, args.epochs, args.steps, args.warmup, args.e2e_chunks, ctx)
+    res = measure(args.workload, wl, args.runs_per_gpu, args.epochs, args.steps, args.warmup, args.e2e_chunks, ctx,
+                  dump_dir=args.dump_outputs)
     line = base_line(args, args.workload, wl, world, _lib.game_layout)
     line.update(res)
     line["parity"] = "green: tests/ -m gpu compare this path with the oracle and the reference's recorded goldens (bit-exact)"
@@ -562,6 +611,9 @@ def run_ours(args):
 
 
 def main():
+    # no bytecode caches in the tree, from this process or the ones it starts (torchrun ranks, reference workers)
+    sys.dont_write_bytecode = True
+    os.environ["PYTHONDONTWRITEBYTECODE"] = "1"
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
     ap.add_argument("--steps", type=int, default=5)
@@ -576,7 +628,13 @@ def main():
     ap.add_argument("--e2e-chunks", type=int, default=None, help="launches the host entry point cuts a step into (default: per workload)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extras", action="store_true", help="skip the c4 / c5 measurements that follow the headline workload")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the headline workload's last timed step computed to DIR/<name>.npy (at most ~50 MB: a fixed sample of the runs)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours")
     wl = WORKLOADS[args.workload]
     if args.global_runs:
         args.runs_per_gpu = args.global_runs // max(1, args.gpus)
