@@ -559,20 +559,26 @@ bool plan_lut2(thrl::Lut2Params* p, bool noisy, size_t elem, int smem_optin, int
   int o = 0;
   p->off_next = o;    o += align_up(2 * J, 16);
   p->off_rowlist = o; o += align_up(2 * (p->NR[0] + p->NR[1]), 16);
-  p->off_lutr = o;    o += J * 16;
   p->off_lutlog = o;  o += J * 32;
+  p->off_lutr = o;
+  p->cta_bytes_lpc = o + J * 16;                                   // qtable_scan_lpc: [J][2] rewards
+  o += align_up(J * 8, 16);
+  p->off_aq = o;      o += align_up((A0 + A1) * 8, 16);            // qtable_scan_lut2: [J] prices, [A0 + A1] quantities
   p->cta_bytes = o;
   o = align_up((p->NR[0] + 2) * A0 * (int)elem, 16);
   p->off_tab1 = o;    o += align_up((p->NR[1] + 2) * A1 * (int)elem, 16);
   p->off_grow = o;    o += align_up(p->NR[0] + p->NR[1] + 4, 16);
   const int nstates = NS + 1 + (noisy ? T : 0);
   p->off_rows = o;    o += align_up(nstates * 4, 16);
-  p->off_gj = o;      o += align_up((NS + 2) * 4, 16);  // lattice states, the initial state, the latest noise step's state
+  {  // lattice states, the initial state, the latest noise step's state; phase D's chunk scratch (+ read-ahead pad) reuses them
+    const int gj = align_up((NS + 2) * 4, 16), scr = thrl::kLut2Chunk * 8 + 16;
+    p->off_gj = o;    o += gj > scr ? gj : scr;
+    p->off_scr = p->off_gj;
+  }
   p->off_nt = o;      o += noisy ? align_up(T, 16) : 0;
   p->off_nrec = o;    o += noisy ? align_up(T * 8, 16) : 0;
   p->off_seq = o;     o += align_up(T + 1, 16);
   p->off_rec = o;     o += align_up(2 * T, 16);
-  p->off_scr = o;     o += thrl::kLut2Chunk * 8 + 16;            // phase D: next-row offsets of one chunk of transitions (+ read-ahead pad)
   {  // phases A-B: pre[T] uint2; phases C-D: olds[T][2] -- disjoint lifetimes, one region
     const int pre = align_up(T * 8, 16), olds = align_up(2 * T * (int)elem, 16);
     p->off_old = o;   o += pre > olds ? pre : olds;
@@ -633,7 +639,7 @@ int launch_lpc_gl(thrl::Lut2Params& p, const DeviceInfo& dev, cudaStream_t strea
   lay.off_eps = o;  o += align_up(GL * 8, 16);
   lay.off_xrow = o; o += align_up(2 * GL * 2, 16);
   lay.warp_bytes = o;
-  int warps = (dev.smem_optin - p.cta_bytes) / lay.warp_bytes;
+  int warps = (dev.smem_optin - p.cta_bytes_lpc) / lay.warp_bytes;
   if (warps < 1) return fail(THRL_ERR_UNSUPPORTED, "lpc: one warp group needs %d B of shared memory", lay.warp_bytes);
   if (warps > thrl::kLpcMaxWarps) warps = thrl::kLpcMaxWarps;
   const long long groups = (p.n_runs + GL / 2 - 1) / (GL / 2);
@@ -643,7 +649,7 @@ int launch_lpc_gl(thrl::Lut2Params& p, const DeviceInfo& dev, cudaStream_t strea
     if (warps < 1) warps = 1;
     grid = (int)((groups + warps - 1) / warps);
   }
-  const size_t smem = (size_t)p.cta_bytes + (size_t)warps * lay.warp_bytes;
+  const size_t smem = (size_t)p.cta_bytes_lpc + (size_t)warps * lay.warp_bytes;
   // compile-time action count for the shapes the reference ships (example_config / configs2: 21 actions)
   const bool a21 = G.agent[0].actions == 21 && G.agent[1].actions == 21;
   auto kern = a21 ? thrl::qtable_scan_lpc<QT, GL, 21> : thrl::qtable_scan_lpc<QT, GL, 0>;

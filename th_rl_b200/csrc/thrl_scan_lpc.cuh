@@ -70,7 +70,7 @@ __global__ void __launch_bounds__(32 * kLpcMaxWarps, 1) qtable_scan_lpc(const __
   __syncthreads();
 
   // ---------------------------------------------------------------- this warp's slot
-  unsigned char* slot = smem + p.cta_bytes + (size_t)warp * lay.warp_bytes;
+  unsigned char* slot = smem + p.cta_bytes_lpc + (size_t)warp * lay.warp_bytes;
   uint8_t* pre_all = slot + lay.off_pre;                           // [T][GL] forced action or 0xFF
   double* eps_sh = reinterpret_cast<double*>(slot + lay.off_eps);  // [GL] current epsilon of every chain
   int16_t* xrow_sh = reinterpret_cast<int16_t*>(slot + lay.off_xrow);  // [2][GL] table rows held in the two extra slots

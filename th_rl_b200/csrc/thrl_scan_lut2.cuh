@@ -5,7 +5,7 @@
 // update) are fixed per joint action.  The host groups joint actions by the encodes of their price into NS "states"
 // (41 for the example config) and lists, per agent, the table rows those states can ever address (the *compact rows*);
 // only those rows (plus the rows of the call's initial price) are staged in shared memory, which more than doubles the
-// number of runs resident per SM.  The f64 lookup values themselves (rewards, reward/T, action/T) are computed by every
+// number of runs resident per SM.  The f64 lookup values themselves (prices, quantities, reward/T, action/T) are computed by every
 // CTA in its prologue with the reference's own formulas.
 //
 // One warp = one run; per epoch:
@@ -18,7 +18,7 @@
 //                 its agent and keeps cell address / reward / (1-alpha)*old in registers; both agents' chains interleaved;
 //                 row max = 1 LDS + 1 CREDUX.MAX; the owning lane stores
 //   E  refresh    greedy cache of the rows that were written (lane = row); epsilon decay; logs / statistics
-// Shared memory per run: compact tables + ~1.7 KB of scratch (DESIGN.md 4.1): 23 runs per SM at the C2 shape.
+// Shared memory per run: compact tables + ~1.6 KB of scratch (DESIGN.md 4.1): 24 runs per SM at the C2 shape.
 #pragma once
 #include "thrl_device.cuh"
 
@@ -54,7 +54,8 @@ struct Lut2Params {
   uint16_t row_list[2][kLut2MaxRows + 3];  // compact row -> table row
   // shared-memory layout
   int cta_bytes, warp_bytes;
-  int off_next, off_rowlist, off_lutr, off_lutlog;  // CTA-shared
+  int cta_bytes_lpc;  // qtable_scan_lpc keeps a [J][2] reward table at off_lutr (this kernel: price per joint action + scaled quantities)
+  int off_next, off_rowlist, off_lutlog, off_lutr, off_aq;  // CTA-shared
   int off_tab1, off_grow, off_rows, off_gj, off_seq, off_rec, off_scr, off_old;  // per warp (tables of agent 0 at 0)
   // demand noise (kNoise): steps whose intercept was redrawn this episode, and what they produced
   int noisy;                // 1: the noisy instantiation runs (state / row arrays hold max_steps more entries)
@@ -105,7 +106,10 @@ __global__ void __launch_bounds__(kNoise ? 32 * kLut2NoiseWarps : 32 * Lut2Warps
   // ---------------------------------------------------------------- CTA-shared lookup tables
   uint16_t* nextS = reinterpret_cast<uint16_t*>(smem + p.off_next);  // joint action -> 4 * next state (byte offset into GJ)
   uint16_t* rowlist = reinterpret_cast<uint16_t*>(smem + p.off_rowlist);  // compact row -> table row, [NR0][NR1]
-  double* lutR = reinterpret_cast<double*>(smem + p.off_lutr);            // [J][2] reward (environments.py:34)
+  // rewards are price(joint) x quantity(action) (environments.py:34): two small tables instead of a [J][2] one, so that a
+  // 24th run fits next to the C2 shape's tables (the product is the same single rounding either way)
+  double* lutP = reinterpret_cast<double*>(smem + p.off_lutr);            // [J] price after the joint action
+  double* lutAq = reinterpret_cast<double*>(smem + p.off_aq);             // [A0 + A1] a/b * scaled action per agent
   double* lutLog = reinterpret_cast<double*>(smem + p.off_lutlog);        // [J][4] r0/T, r1/T, x0/T, x1/T (trainer.py:65-66)
   {
     const double ab = __ddiv_rn(G.a, G.b);
@@ -118,13 +122,16 @@ __global__ void __launch_bounds__(kNoise ? 32 * kLut2NoiseWarps : 32 * Lut2Warps
       const double pn = __dsub_rn(G.a, __dmul_rn(G.b, Q));
       const double price = pn > 0.0 ? pn : (pn != pn ? pn : 0.0);
       const double r0 = __dmul_rn(price, aq0), r1 = __dmul_rn(price, aq1);
-      lutR[2 * j] = r0;
-      lutR[2 * j + 1] = r1;
+      lutP[j] = price;
       lutLog[4 * j + 0] = __ddiv_rn(r0, (double)T);
       lutLog[4 * j + 1] = __ddiv_rn(r1, (double)T);
       lutLog[4 * j + 2] = __ddiv_rn(x0, (double)T);
       lutLog[4 * j + 3] = __ddiv_rn(x1, (double)T);
       nextS[j] = (uint16_t)(4u * p.next_state[j]);
+    }
+    for (int k = threadIdx.x; k < A0 + A1; k += blockDim.x) {
+      const ThrlAgentSpec& sa = G.agent[k < A0 ? 0 : 1];
+      lutAq[k] = __dmul_rn(ab, scale_action(k < A0 ? k : k - A0, sa.actions, sa.action_lo, sa.action_hi));
     }
     for (int c = threadIdx.x; c < NR0 + NR1; c += blockDim.x)
       rowlist[c] = c < NR0 ? p.row_list[0][c] : p.row_list[1][c - NR0];
@@ -142,7 +149,8 @@ __global__ void __launch_bounds__(kNoise ? 32 * kLut2NoiseWarps : 32 * Lut2Warps
   uint16_t* rec = reinterpret_cast<uint16_t*>(slot + p.off_rec);     // [T] k0 | k1<<8
   uint8_t* seq = slot + p.off_seq;                                   // [T+1] state before step t (rebuilt lane-parallel)
   uint2* pre = reinterpret_cast<uint2*>(slot + p.off_old);           // [T] (keep mask, forced value) byte pairs (phases A-B; olds in C-D)
-  // phase D chunk: [kLut2Chunk] uint2 = next-row byte offsets of (agent 0, agent 1) for the transitions being applied
+  // phase D chunk: [kLut2Chunk] uint2 = next-row byte offsets of (agent 0, agent 1) for the transitions being applied.  It
+  // shares its bytes with GJ: phases C-D never read GJ, and phase E rebuilds it (GJ[NS+1] is written before it is read)
   unsigned char* chunk = slot + p.off_scr;
   QT* olds = reinterpret_cast<QT*>(slot + p.off_old);                // [T][2] stale old values of the batch (agents.py:67)
   uint8_t* nT = slot + p.off_nt;                                     // kNoise: [T] step of the k-th noise event of the episode
@@ -426,8 +434,8 @@ __global__ void __launch_bounds__(kNoise ? 32 * kLut2NoiseWarps : 32 * Lut2Warps
             p.trace_rewards[(step0 + t) * 2] = __dmul_rn(nrec[ks], __dmul_rn(ab, scale_action(k0, A0, G.agent[0].action_lo, G.agent[0].action_hi)));
             p.trace_rewards[(step0 + t) * 2 + 1] = __dmul_rn(nrec[ks], __dmul_rn(ab, scale_action(k1, A1, G.agent[1].action_lo, G.agent[1].action_hi)));
           } else if (p.trace_rewards) {
-            p.trace_rewards[(step0 + t) * 2] = lutR[2 * joint];
-            p.trace_rewards[(step0 + t) * 2 + 1] = lutR[2 * joint + 1];
+            p.trace_rewards[(step0 + t) * 2] = __dmul_rn(lutP[joint], lutAq[k0]);
+            p.trace_rewards[(step0 + t) * 2 + 1] = __dmul_rn(lutP[joint], lutAq[A0 + k1]);
           }
           if (p.trace_prices && ks >= 0) {
             p.trace_prices[step0 + t] = nrec[ks];
@@ -470,7 +478,7 @@ __global__ void __launch_bounds__(kNoise ? 32 * kLut2NoiseWarps : 32 * Lut2Warps
         const int cu = ag ? (int)(rw >> 24) : (int)((rw >> 8) & 0xff), cn = ag ? (int)(rn >> 24) : (int)((rn >> 8) & 0xff);
         row_off = (uint32_t)(cn * Aa) * (uint32_t)sizeof(QT);
         cell_addr = (ag ? tab1_off : tab0_off) + (uint32_t)(cu * Aa + k) * (uint32_t)sizeof(QT);
-        double rew = lutR[2 * joint + ag];
+        double rew = __dmul_rn(lutP[joint], lutAq[ag ? A0 + k : k]);
         if (kNoise && seq[j + 1] > NS) {  // a noise step: reward = its price x the agent's quantity (environments.py:34)
           const ThrlAgentSpec& sa = G.agent[ag];
           rew = __dmul_rn(nrec[(int)seq[j + 1] - NS - 1], __dmul_rn(__ddiv_rn(G.a, G.b), scale_action(k, Aa, sa.action_lo, sa.action_hi)));
