@@ -551,29 +551,41 @@ __global__ void __launch_bounds__(kNoise ? 32 * kLut2NoiseWarps : 32 * Lut2Warps
 
       // ---- E: refresh the greedy cache of written rows, then the per-state greedy pairs
       {
-        // lane = compact row: every lane scans one written row left to right (first maximum, agents.py:88); rows of
-        // distinct lanes start A elements apart, so for odd A the scan is bank-conflict-free
-        auto refresh = [&](const QT* tab, int A, int NRa, uint8_t* gr, unsigned wa, unsigned wb, bool all) {
-          wa = __reduce_or_sync(kFull, wa);
-          wb = __reduce_or_sync(kFull, wb);
-          const bool every = __any_sync(kFull, all);
-          for (int c = lane; c < NRa + 2; c += 32) {
-            const bool d = c < 32 ? (wa >> c) & 1u : (c < 64 ? (wb >> (c - 32)) & 1u : every);
-            if (d) {
-              const QT* row = tab + c * A;
-              QT m = row[0];
-              int g = 0;
+        // lane = written row: a lane scans one row left to right for its first maximum (agents.py:88)
+        auto scan_row = [&](const QT* row, int A) -> int {
+          QT m = row[0];
+          int g = 0;
 #pragma unroll 4
-              for (int k = 1; k < A; ++k) {
-                const QT v = row[k];
-                if (v > m) { m = v; g = k; }
-              }
-              gr[c] = (uint8_t)g;
-            }
+          for (int k = 1; k < A; ++k) {
+            const QT v = row[k];
+            if (v > m) { m = v; g = k; }
           }
+          return g;
         };
-        refresh(tab0, A0, NR0, grow, dirty0a, dirty0b, dirty_all0);
-        refresh(tab1, A1, NR1, grow + NR0 + 2, dirty1a, dirty1b, dirty_all1);
+        // Rows 0..63 of both agents: the written ones (masks of C) are listed in the olds scratch, which D is done with,
+        // agent 0's first.  A batch writes at most L0 + L1 <= 2T rows and olds holds 2T elements, so the list fits; one pass
+        // of the warp covers 32 written rows of the two agents together (typically all of them) instead of two passes over
+        // every compact row of each agent.
+        const unsigned w0a = __reduce_or_sync(kFull, dirty0a), w0b = __reduce_or_sync(kFull, dirty0b);
+        const unsigned w1a = __reduce_or_sync(kFull, dirty1a), w1b = __reduce_or_sync(kFull, dirty1b);
+        const unsigned below = (1u << lane) - 1u;
+        const int n0a = __popc(w0a), n0 = n0a + __popc(w0b), n1a = n0 + __popc(w1a), nd = n1a + __popc(w1b);
+        uint8_t* dlist = reinterpret_cast<uint8_t*>(olds);
+        if ((w0a >> lane) & 1u) dlist[__popc(w0a & below)] = (uint8_t)lane;
+        if ((w0b >> lane) & 1u) dlist[n0a + __popc(w0b & below)] = (uint8_t)(32 + lane);
+        if ((w1a >> lane) & 1u) dlist[n0 + __popc(w1a & below)] = (uint8_t)lane;
+        if ((w1b >> lane) & 1u) dlist[n1a + __popc(w1b & below)] = (uint8_t)(32 + lane);
+        __syncwarp();
+        for (int i = lane; i < nd; i += 32) {  // selects, not a branch: lanes of both agents scan together
+          const bool ag = i >= n0;
+          const int c = dlist[i], A = ag ? A1 : A0;
+          grow[(ag ? NR0 + 2 : 0) + c] = (uint8_t)scan_row((ag ? tab1 : tab0) + c * A, A);
+        }
+        // rows from 64 on are not in the masks: all of them when the batch wrote any
+        if (__any_sync(kFull, dirty_all0))
+          for (int c = 64 + lane; c < NR0 + 2; c += 32) grow[c] = (uint8_t)scan_row(tab0 + c * A0, A0);
+        if (__any_sync(kFull, dirty_all1))
+          for (int c = 64 + lane; c < NR1 + 2; c += 32) grow[NR0 + 2 + c] = (uint8_t)scan_row(tab1 + c * A1, A1);
         __syncwarp();
         if (kNoise && sig4 > 4u * (uint32_t)NS) {  // the episode ended on a noise step: its state becomes the next episode's state NS
           if (lane == 0) rowsW[NS] = rowsW[NS + nK];
