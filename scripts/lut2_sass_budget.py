@@ -6,7 +6,7 @@ SASS alone (CPU only; no profiler needed).
 The kernel is disassembled with line info (`cuobjdump -xelf`, `nvdisasm -gi`).  Every instruction is attributed to the line
 of thrl_scan_lut2.cuh it comes from (the call site, for inlined helpers), and the line to a phase by the markers in the
 source (an instruction from a line of the kernel's prologue, a value re-derived inside a loop, goes with the one before it):
-  A       draws (Philox)                       seq     rebuild of the state sequence from the action record
+  A       draws (Philox)                       seq     rebuild of the state sequence (noisy instantiation only: 0 here)
   B       rollout                              C       snapshot (old values, visit counters, dirty masks)
   expand  D's per-chunk expansion + prologue   D       D's inner loop (one transition of each agent per iteration)
   E       greedy refresh, greedy-pair cache    stats   epsilon decay, logs, statistics
@@ -68,6 +68,7 @@ def loop_trips(text, s):
         (r"for \(int t = lane; t < T; t \+= 32\)", math.ceil(T / 32)),          # A (and traces)
         (r"for \(int n2 = T >> 1", T / 2 / 2),                                  # B, pairs, unroll 2
         (r"for \(int t = lane; t <= T; t \+= 32\)", math.ceil((T + 1) / 32)),   # seq
+        (r"for \(int j = T - L1 \+ lane; j < T; j \+= 32\) reinterpret_cast", 0),  # C, unequal batches only (none at C2)
         (r"for \(int j = T - L0 \+ lane|for \(int j = T - L1 \+ lane", math.ceil(L / 32)),  # C, one agent per loop
         (r"for \(int j = T - \(L0 > L1", math.ceil(L / 32)),                   # C, both agents per step
         (r"for \(int c0 = 0; c0 < L0; c0 \+= kLut2Chunk\)", s["chunks"]),      # D chunks

@@ -40,6 +40,18 @@ __device__ __forceinline__ double u53(uint32_t hi, uint32_t lo) {
 
 // 32-bit uniform in [0,1) for the exploration test (exact: integer < 2^32 times 2^-32)
 __device__ __forceinline__ double u32_unit(uint32_t x) { return __dmul_rn((double)x, 1.0 / 4294967296.0); }
+// The same test in integers: u32_unit(x) < eps  <=>  x < u32_unit_threshold(eps), for every x and every eps (NaN and
+// infinities included).  Proof: u32_unit(x) is x * 2^-32 exactly, and y = eps * 2^32 is exact in f64 (a power-of-two
+// scaling; +-inf on overflow, which still orders correctly), so u32_unit(x) < eps <=> x < y.  For an integer x,
+// x < y <=> x < ceil(y).  y <= 0 or NaN: no x qualifies (threshold 0); y > 2^32 - 1: every x does (threshold 2^32, hence
+// 64 bits); otherwise ceil(y) lies in [1, 2^32 - 1].  Computed once per epsilon, it replaces a convert, a multiply and a
+// compare in f64 per draw by one integer compare.
+__device__ __forceinline__ unsigned long long u32_unit_threshold(double eps) {
+  const double y = __dmul_rn(eps, 4294967296.0);
+  if (!(y > 0.0)) return 0ull;
+  if (y > 4294967295.0) return 1ull << 32;
+  return (unsigned long long)ceil(y);
+}
 
 // ---------------------------------------------------------------- state encodes (th_rl/agents.py:47-49)
 // float32 encode of the state handed to sample_action (trainer.py:53): rint_f32(f32(p) / f32(max_state) * f32(states))

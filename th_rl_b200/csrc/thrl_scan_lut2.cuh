@@ -9,16 +9,17 @@
 // CTA in its prologue with the reference's own formulas.
 //
 // One warp = one run; per epoch:
-//   A  draws      lane-parallel Philox (or replay streams) -> per-step forced actions (epsilon is frozen in an episode)
+//   A  draws      lane-parallel Philox (or replay streams) -> per-step forced actions (epsilon is frozen in an episode;
+//                 the exploration test is an integer compare against a per-epoch threshold)
 //   B  rollout    sequential, two steps per iteration: state -> greedy pair (cached per state) -> forced override ->
 //                 joint action -> next state; log sums on lanes 0-3
 //   C  snapshot   lane-parallel: stale old value of every transition of the batch (agents.py:67), visit counters (RED),
-//                 dirty-row masks
+//                 dirty-row masks; the state before a step is derived from the action record (no state sequence is kept)
 //   D  update     sequential (agents.py:68-76) in chunks of 16 transitions; lane i of a half-warp expands transition i of
 //                 its agent and keeps cell address / reward / (1-alpha)*old in registers; both agents' chains interleaved;
 //                 row max = 1 LDS + 1 CREDUX.MAX; the owning lane stores
 //   E  refresh    greedy cache of the rows that were written (lane = row); epsilon decay; logs / statistics
-// Shared memory per run: compact tables + ~1.6 KB of scratch (DESIGN.md 4.1): 24 runs per SM at the C2 shape.
+// Shared memory per run: compact tables + ~1.5 KB of scratch (DESIGN.md 4.1): 24 runs per SM at the C2 shape.
 #pragma once
 #include "thrl_device.cuh"
 
@@ -147,7 +148,7 @@ __global__ void __launch_bounds__(kNoise ? 32 * kLut2NoiseWarps : 32 * Lut2Warps
   unsigned char* GJb = slot + p.off_gj;                              // [NS+1] u32: state -> greedy g0 | g1<<8
   uint32_t* GJ = reinterpret_cast<uint32_t*>(GJb);
   uint16_t* rec = reinterpret_cast<uint16_t*>(slot + p.off_rec);     // [T] k0 | k1<<8
-  uint8_t* seq = slot + p.off_seq;                                   // [T+1] state before step t (rebuilt lane-parallel)
+  uint8_t* seq = slot + p.off_seq;                                   // kNoise: [T+1] state before step t (rebuilt lane-parallel)
   uint2* pre = reinterpret_cast<uint2*>(slot + p.off_old);           // [T] (keep mask, forced value) byte pairs (phases A-B; olds in C-D)
   // phase D chunk: [kLut2Chunk] uint2 = next-row byte offsets of (agent 0, agent 1) for the transitions being applied.  It
   // shares its bytes with GJ: phases C-D never read GJ, and phase E rebuilds it (GJ[NS+1] is written before it is read)
@@ -175,17 +176,15 @@ __global__ void __launch_bounds__(kNoise ? 32 * kLut2NoiseWarps : 32 * Lut2Warps
     uint32_t* cnt0 = p.counter ? p.counter + r * G.run_stride : nullptr;
     uint32_t* cnt1 = cnt0 ? cnt0 + G.agent[1].table_offset : nullptr;
     const uint32_t gid = (uint32_t)(p.run_id0 + r);
-    double alpha0, gamma0, epsend0, epsstep0, alpha1, gamma1, epsend1, epsstep1;
-    if (p.hp) {
-      const double* h = p.hp + r * 8;
-      alpha0 = h[0]; gamma0 = h[1]; epsend0 = h[2]; epsstep0 = h[3];
-      alpha1 = h[4]; gamma1 = h[5]; epsend1 = h[6]; epsstep1 = h[7];
-    } else {
-      alpha0 = G.agent[0].alpha; gamma0 = G.agent[0].gamma; epsend0 = G.agent[0].eps_end; epsstep0 = G.agent[0].eps_step;
-      alpha1 = G.agent[1].alpha; gamma1 = G.agent[1].gamma; epsend1 = G.agent[1].eps_end; epsstep1 = G.agent[1].eps_step;
-    }
-    const double oma0 = __dsub_rn(1.0, alpha0), oma1 = __dsub_rn(1.0, alpha1);
-    double alpha_h = hi_half ? alpha1 : alpha0, gamma_h = hi_half ? gamma1 : gamma0, oma_h = hi_half ? oma1 : oma0;
+    // the run's hyper-parameters of agent ag: alpha, gamma, eps_end, eps_step (k = 0..3).  They are read where they are used
+    // (per half once per run; epsilon decay once per epoch) instead of being held across the epoch loop: ten f64 values
+    // would take 20 of the 80 registers that the update and its chunk expansion need.
+    auto hparam = [&](int ag, int k) -> double {
+      if (p.hp) return __ldg(p.hp + r * 8 + ag * 4 + k);
+      const ThrlAgentSpec& s = G.agent[ag];
+      return k == 0 ? s.alpha : k == 1 ? s.gamma : k == 2 ? s.eps_end : s.eps_step;
+    };
+    double alpha_h = hparam(hi_half, 0), gamma_h = hparam(hi_half, 1), oma_h = __dsub_rn(1.0, alpha_h);
     asm volatile("" : "+d"(alpha_h), "+d"(gamma_h), "+d"(oma_h));  // keep the selected values live (no re-selection in the loops)
     double eps0 = p.eps[r * 2], eps1 = p.eps[r * 2 + 1];
     const double price_in = p.price[r];
@@ -259,13 +258,14 @@ __global__ void __launch_bounds__(kNoise ? 32 * kLut2NoiseWarps : 32 * Lut2Warps
 
       // ---- A: draws (agents.py:81-82), lane-parallel over the steps of the episode.
       //      pre[t] = (keep, forced): action pair = (greedy pair & keep) | forced
+      const unsigned long long thr0 = u32_unit_threshold(eps0), thr1 = u32_unit_threshold(eps1);  // u32_unit(x) < eps <=> x < thr
       for (int t = lane; t < T; t += 32) {
         int f0, f1;
         if (rng_mode == THRL_RNG_PHILOX) {
           uint32_t x[4];
           philox4x32_10(gid, eabs, (uint32_t)t, kStreamAct << 16, key0, key1, x);
-          f0 = u32_unit(x[0]) < eps0 ? (int)__umulhi(x[1], (uint32_t)A0) : -1;
-          f1 = u32_unit(x[2]) < eps1 ? (int)__umulhi(x[3], (uint32_t)A1) : -1;
+          f0 = x[0] < thr0 ? (int)__umulhi(x[1], (uint32_t)A0) : -1;
+          f1 = x[2] < thr1 ? (int)__umulhi(x[3], (uint32_t)A1) : -1;
         } else if (rng_mode == THRL_RNG_REPLAY_DRAWS) {
           const double2 u = *reinterpret_cast<const double2*>(p.replay_u + (step0 + t) * 2);
           const int2 v = *reinterpret_cast<const int2*>(p.replay_ra + (step0 + t) * 2);
@@ -411,17 +411,25 @@ __global__ void __launch_bounds__(kNoise ? 32 * kLut2NoiseWarps : 32 * Lut2Warps
         last_k = (int)kk;
       }
       __syncwarp();
-      // states before every step, rebuilt lane-parallel from the action record
-      for (int t = lane; t <= T; t += 32) {
-        uint32_t s4 = sig4_start;
-        if (t > 0) { const uint32_t kk = rec[t - 1]; s4 = nextS[__dp4a(kk, dp_b, 0u)]; }
-        seq[t] = (uint8_t)(s4 >> 2);
-      }
-      __syncwarp();
-      if (kNoise) {  // the state after a noise step is that step's extra state
+      if (kNoise) {
+        // states before every step, rebuilt lane-parallel from the action record; the state after a noise step is that
+        // step's extra state
+        for (int t = lane; t <= T; t += 32) {
+          uint32_t s4 = sig4_start;
+          if (t > 0) { const uint32_t kk = rec[t - 1]; s4 = nextS[__dp4a(kk, dp_b, 0u)]; }
+          seq[t] = (uint8_t)(s4 >> 2);
+        }
+        __syncwarp();
         for (int k = lane; k < nK; k += 32) seq[nT[k] + 1] = (uint8_t)(NS + 1 + k);
         __syncwarp();
       }
+      // compact rows of the state before step j (rowsW entry).  Noise-free, that state is where step j-1 led,
+      // nextS[joint(rec[j-1])], and the episode's start state for j = 0; nextS holds 4 x state, the entry's byte offset.
+      auto rows_before = [&](int j) -> uint32_t {
+        if (kNoise) return rowsW[seq[j]];
+        const uint32_t led = nextS[__dp4a((uint32_t)rec[j > 0 ? j - 1 : 0], dp_b, 0u)];  // loads, then a select: no branch
+        return *reinterpret_cast<const uint32_t*>(reinterpret_cast<const unsigned char*>(rowsW) + (j > 0 ? led : sig4_start));
+      };
 
       // optional per-step traces (parity runs only), lane-parallel
       if (p.trace_actions || p.trace_rewards || p.trace_prices) {
@@ -454,28 +462,52 @@ __global__ void __launch_bounds__(kNoise ? 32 * kLut2NoiseWarps : 32 * Lut2Warps
       //      which keeps the per-run scratch small (more runs resident per SM).
       unsigned dirty0a = 0, dirty0b = 0, dirty1a = 0, dirty1b = 0;  // written compact rows 0..63 of each agent
       bool dirty_all0 = false, dirty_all1 = false;
+      // Agent 1's pass reads the rows word of each of its steps from the olds slot it then fills.  With equal batches (the
+      // usual case) agent 0's pass visits the same steps and leaves it there, so the state is derived once per step.
+      const bool pass_rows = L0 == L1;
+      if (!pass_rows)
+        for (int j = T - L1 + lane; j < T; j += 32) reinterpret_cast<uint32_t*>(olds + 2 * (j - (T - L1)) + 1)[0] = rows_before(j);
       for (int j = T - L0 + lane; j < T; j += 32) {
-        const int k = rec[j] & 0xff, cu = (rowsW[seq[j]] >> 8) & 0xff;
-        olds[2 * (j - (T - L0))] = tab0[cu * A0 + k];
+        const uint32_t rw = rows_before(j);
+        const int k = rec[j] & 0xff, cu = (rw >> 8) & 0xff, jj = j - (T - L0);
+        olds[2 * jj] = tab0[cu * A0 + k];
+        if (pass_rows) reinterpret_cast<uint32_t*>(olds + 2 * jj + 1)[0] = rw;
         if (cnt0) atomicAdd(cnt0 + (size_t)table_row0(cu) * G.agent[0].row_stride + k, 1u);  // agents.py:76
         if (cu < 32) dirty0a |= 1u << cu; else if (cu < 64) dirty0b |= 1u << (cu - 32); else dirty_all0 = true;
       }
       for (int j = T - L1 + lane; j < T; j += 32) {
-        const int k = rec[j] >> 8, cu = rowsW[seq[j]] >> 24;
+        const int k = rec[j] >> 8, cu = reinterpret_cast<const uint32_t*>(olds + 2 * (j - (T - L1)) + 1)[0] >> 24;
         olds[2 * (j - (T - L1)) + 1] = tab1[cu * A1 + k];
         if (cnt1) atomicAdd(cnt1 + (size_t)table_row1(cu) * G.agent[1].row_stride + k, 1u);
         if (cu < 32) dirty1a |= 1u << cu; else if (cu < 64) dirty1b |= 1u << (cu - 32); else dirty_all1 = true;
       }
       __syncwarp();
 
-      // chunk expansion, lane-parallel: transition jj of agent ag -> (next-row byte offset, cell address, reward, (1-alpha)*old)
-      auto expand = [&](int jj, int ag, int La, double oma, uint32_t& row_off, uint32_t& cell_addr, double2& v) {
+      // chunk expansion, lane-parallel: transition jj of agent ag -> (next-row byte offset, cell address, reward, (1-alpha)*old).
+      // Noise-free, every lane calls it, a lane of half h taking transition jj = c0 + (lane & 15) (clamped to the batch: lanes
+      // past its end repeat the last transition, and their countdown never reaches the store).  It loads the compact rows
+      // after its step only: the rows before it are the rows after the previous transition, held by the lane below, and for
+      // the first lane of a half they are carried over from the previous chunk (rw_carry: rows before transition c0 on entry,
+      // before c0 + 16 on return).
+      auto expand = [&](int jj, int ag, int La, double oma, uint32_t& rw_carry, uint32_t& row_off, uint32_t& cell_addr,
+                        double2& v) {
         const int j = T - La + jj;
-        const uint32_t rw = rowsW[seq[j]], rn = rowsW[seq[j + 1]];
         const uint32_t kk = rec[j];
+        uint32_t rw, rn;
+        if (kNoise) {
+          rw = rowsW[seq[j]];
+          rn = rowsW[seq[j + 1]];
+        } else {
+          rn = *reinterpret_cast<const uint32_t*>(reinterpret_cast<const unsigned char*>(rowsW) + nextS[__dp4a(kk, dp_b, 0u)]);
+          const uint32_t below = __shfl_up_sync(kFull, rn, 1, kLut2Chunk);
+          rw = (lane & (kLut2Chunk - 1)) ? below : rw_carry;
+          rw_carry = __shfl_sync(kFull, rn, kLut2Chunk - 1);
+        }
         const int joint = (int)__dp4a(kk, dp_b, 0u);
-        const int Aa = ag ? A1 : A0, k = ag ? (int)(kk >> 8) : (int)(kk & 0xff);
-        const int cu = ag ? (int)(rw >> 24) : (int)((rw >> 8) & 0xff), cn = ag ? (int)(rn >> 24) : (int)((rn >> 8) & 0xff);
+        // the agent's bytes: k = byte ag of kk, update rows = byte 1 + 2 ag of a rows word (one PRMT each)
+        const uint32_t sel_row = ag ? 0x4443u : 0x4441u;
+        const int Aa = ag ? A1 : A0, k = (int)__byte_perm(kk, 0u, ag ? 0x4441u : 0x4440u);
+        const int cu = (int)__byte_perm(rw, 0u, sel_row), cn = (int)__byte_perm(rn, 0u, sel_row);
         row_off = (uint32_t)(cn * Aa) * (uint32_t)sizeof(QT);
         cell_addr = (ag ? tab1_off : tab0_off) + (uint32_t)(cu * Aa + k) * (uint32_t)sizeof(QT);
         double rew = __dmul_rn(lutP[joint], lutAq[ag ? A0 + k : k]);
@@ -484,6 +516,7 @@ __global__ void __launch_bounds__(kNoise ? 32 * kLut2NoiseWarps : 32 * Lut2Warps
           rew = __dmul_rn(nrec[(int)seq[j + 1] - NS - 1], __dmul_rn(__ddiv_rn(G.a, G.b), scale_action(k, Aa, sa.action_lo, sa.action_hi)));
         }
         v = make_double2(rew, __dmul_rn(oma, (double)olds[2 * jj + ag]));
+        asm volatile("" : "+d"(v.x), "+d"(v.y), "+r"(cell_addr));  // computed here, not sunk into the update's loop
       };
 
       // ---- D: the sequential pass (agents.py:68-76).  The two agents' chains are independent: both rows are loaded
@@ -499,11 +532,13 @@ __global__ void __launch_bounds__(kNoise ? 32 * kLut2NoiseWarps : 32 * Lut2Warps
         // two next-row offsets of every transition go through shared memory (one uniform 8-byte load per iteration).  The
         // row maxima are warp reductions, so every lane evaluates :72-74 and the lane that owns transition j stores.
         const int li = lane & (kLut2Chunk - 1);
+        uint32_t rw_carry = kNoise ? 0u : rows_before(T - L0);
         for (int c0 = 0; c0 < L0; c0 += kLut2Chunk) {
           const int n = L0 - c0 < kLut2Chunk ? L0 - c0 : kLut2Chunk;
           uint32_t row_off = 0, cell_addr = 0;
           double2 v = make_double2(0.0, 0.0);
-          if (li < n) expand(c0 + li, lane >> 4, L0, oma_h, row_off, cell_addr, v);
+          if (!kNoise) expand(min(c0 + li, L0 - 1), lane >> 4, L0, oma_h, rw_carry, row_off, cell_addr, v);
+          else if (li < n) expand(c0 + li, lane >> 4, L0, oma_h, rw_carry, row_off, cell_addr, v);
           const uint32_t other = __shfl_xor_sync(kFull, row_off, 16);
           if (lane < n) *reinterpret_cast<uint2*>(smem + chunk_off + lane * 8) = make_uint2(row_off, other);
           __syncwarp();
@@ -528,15 +563,16 @@ __global__ void __launch_bounds__(kNoise ? 32 * kLut2NoiseWarps : 32 * Lut2Warps
       } else {
         for (int ag = 0; ag < 2; ++ag) {
           const int La = ag ? L1 : L0;
-          const double alpha = ag ? alpha1 : alpha0, gamma = ag ? gamma1 : gamma0;
+          const double alpha = hparam(ag, 0), gamma = hparam(ag, 1), oma = __dsub_rn(1.0, alpha);
+          uint32_t rw_carry = kNoise || La == 0 ? 0u : rows_before(T - La);
           for (int c0 = 0; c0 < La; c0 += kLut2Chunk) {
             const int n = La - c0 < kLut2Chunk ? La - c0 : kLut2Chunk;
             uint32_t row_off = 0, cell_addr = 0;
             double2 v = make_double2(0.0, 0.0);
-            if (lane < n) {
-              expand(c0 + lane, ag, La, ag ? oma1 : oma0, row_off, cell_addr, v);
-              *reinterpret_cast<uint32_t*>(smem + chunk_off + lane * 8) = row_off;
-            }
+            const int li = lane & (kLut2Chunk - 1);  // lanes 16-31 repeat lanes 0-15 and never store
+            if (!kNoise) expand(min(c0 + li, La - 1), ag, La, oma, rw_carry, row_off, cell_addr, v);
+            else if (lane < n) expand(c0 + lane, ag, La, oma, rw_carry, row_off, cell_addr, v);
+            if (lane < n) *reinterpret_cast<uint32_t*>(smem + chunk_off + lane * 8) = row_off;
             __syncwarp();
             for (int j = 0; j < n; ++j) {
               const uint32_t ro = *reinterpret_cast<const uint32_t*>(smem + chunk_off + j * 8);
@@ -601,8 +637,11 @@ __global__ void __launch_bounds__(kNoise ? 32 * kLut2NoiseWarps : 32 * Lut2Warps
         }
       }
       // epsilon decay, every epoch (agents.py:78)
-      eps0 = __dadd_rn(epsend0, __dmul_rn(__dsub_rn(eps0, epsend0), epsstep0));
-      eps1 = __dadd_rn(epsend1, __dmul_rn(__dsub_rn(eps1, epsend1), epsstep1));
+      {
+        const double epsend0 = hparam(0, 2), epsstep0 = hparam(0, 3), epsend1 = hparam(1, 2), epsstep1 = hparam(1, 3);
+        eps0 = __dadd_rn(epsend0, __dmul_rn(__dsub_rn(eps0, epsend0), epsstep0));
+        eps1 = __dadd_rn(epsend1, __dmul_rn(__dsub_rn(eps1, epsend1), epsstep1));
+      }
       // logs and statistics: lane 0,1 = rewards_log[e, 0..1], lane 2,3 = actions_log[e, 0..1]
       if (lane < 4) {
         const int ag = lane & 1;
