@@ -209,14 +209,18 @@ def _sweep_hp(rng, R, n):
     return hp
 
 
-def _philox_case(cfg, R, E, dtype, seed, run_id0=0, hp=False, chunks=None):
+def _philox_case(cfg, R, E, dtype, seed, run_id0=0, hp=False, chunks=None, state=None):
+    """hp: True draws per-run hyper-parameters, an [R, n, 4] array gives them.  state: (q0, eps0, p0) to start from instead
+    of the library's initial state."""
     torch, oracle, engine = _mods()
     game = oracle.layout(cfg)
     n = game.n_agents
     rng = np.random.default_rng(seed)
-    hpa = _sweep_hp(rng, R, n) if hp else None
+    hpa = hp if isinstance(hp, np.ndarray) else (_sweep_hp(rng, R, n) if hp else None)
     q0, c0, eps0, p0, *rest = oracle.init(game, R, seed=seed, run_id0=run_id0, dtype=dtype, hp=hpa,
                                           eps0=abi.eps0_from_config(cfg))
+    if state is not None:
+        q0, eps0, p0 = state
     mlp0 = rest[0] if rest else None
     ref = oracle.scan(game, q0, eps0, p0, E, hp=hpa, seed=seed, run_id0=run_id0, stats=True, trace=True, n_threads=0, mlp=mlp0)
     tdt = torch.float64 if dtype == np.float64 else torch.float32
@@ -628,30 +632,39 @@ def _two_agent_cfg(T, a0, a1, env=None):
             "training": dict(print_freq=500, epochs=3)}
 
 
-@pytest.mark.parametrize("case", ["odd_T", "short_T", "partial_chunks", "unequal_batches", "one_never_fires", "unequal_actions",
-                                  "wide_actions", "noise_all", "noise_most", "noise_rare"])
+TWO_AGENT_CASES = {
+    "odd_T": _two_agent_cfg(33, dict(min_memory=33, capacity=500), dict(min_memory=20, capacity=500)),
+    "short_T": _two_agent_cfg(7, dict(min_memory=5, capacity=50), dict(min_memory=7, capacity=50)),
+    "partial_chunks": _two_agent_cfg(100, dict(min_memory=50, capacity=53), dict(min_memory=10, capacity=53)),
+    "unequal_batches": _two_agent_cfg(60, dict(min_memory=10, capacity=17), dict(min_memory=40, capacity=45)),
+    "one_never_fires": _two_agent_cfg(40, dict(min_memory=30, capacity=40), dict(min_memory=100, capacity=50)),
+    "unequal_actions": _two_agent_cfg(50, dict(actions=5, min_memory=50, capacity=500), dict(actions=9, states=37, min_memory=50, capacity=500)),
+    "wide_actions": _two_agent_cfg(30, dict(actions=40, states=60, min_memory=30), dict(actions=21, min_memory=30)),
+    # demand noise on the specialised kernel: every step a noise step (odd episode length: the rollout is single steps only),
+    # most steps (runs of consecutive noise steps, episodes that end on one), and the environment's default 5 %
+    "noise_all": _two_agent_cfg(33, dict(min_memory=33, capacity=500), dict(min_memory=20, capacity=500), env=dict(noise_prob=1.0)),
+    "noise_most": _two_agent_cfg(100, dict(min_memory=50, capacity=53), dict(min_memory=10, capacity=53), env=dict(noise_prob=0.6)),
+    "noise_rare": _two_agent_cfg(100, dict(), dict(actions=9, states=37), env=dict(noise_prob=0.05)),
+    "T1": _two_agent_cfg(1, dict(min_memory=1, capacity=1), dict(min_memory=1, capacity=1)),
+    "T2": _two_agent_cfg(2, dict(min_memory=2, capacity=2), dict(min_memory=2, capacity=2)),
+    "L16": _two_agent_cfg(48, dict(min_memory=16, capacity=16), dict(min_memory=16, capacity=16)),
+    "L17": _two_agent_cfg(48, dict(min_memory=17, capacity=17), dict(min_memory=17, capacity=17)),
+    "L32": _two_agent_cfg(48, dict(min_memory=32, capacity=32), dict(min_memory=32, capacity=32)),
+}
+
+
+@pytest.mark.parametrize("case", list(TWO_AGENT_CASES))
 def test_two_agent_edge_shapes_match_oracle(case, kernel_choice):
     """Shapes that exercise the corners of the specialised 2-agent kernel: odd / tiny episode lengths (rollout tail, a single
     partial update chunk), batches that are not a multiple of the 16-transition chunk, agents whose batches differ in
-    length (separate update loops), an agent whose buffer never reaches min_memory, unequal and > 32-column action grids."""
+    length (separate update loops), an agent whose buffer never reaches min_memory, unequal and > 32-column action grids;
+    one-step and two-step episodes, batches of exactly one update chunk (its read-ahead reaches the pad), one more, and
+    exactly two chunks."""
     from th_rl_b200 import _lib
-    cfg = {
-        "odd_T": _two_agent_cfg(33, dict(min_memory=33, capacity=500), dict(min_memory=20, capacity=500)),
-        "short_T": _two_agent_cfg(7, dict(min_memory=5, capacity=50), dict(min_memory=7, capacity=50)),
-        "partial_chunks": _two_agent_cfg(100, dict(min_memory=50, capacity=53), dict(min_memory=10, capacity=53)),
-        "unequal_batches": _two_agent_cfg(60, dict(min_memory=10, capacity=17), dict(min_memory=40, capacity=45)),
-        "one_never_fires": _two_agent_cfg(40, dict(min_memory=30, capacity=40), dict(min_memory=100, capacity=50)),
-        "unequal_actions": _two_agent_cfg(50, dict(actions=5, min_memory=50, capacity=500), dict(actions=9, states=37, min_memory=50, capacity=500)),
-        "wide_actions": _two_agent_cfg(30, dict(actions=40, states=60, min_memory=30), dict(actions=21, min_memory=30)),
-        # demand noise on the specialised kernel: every step a noise step (odd episode length: the rollout is single steps only),
-        # most steps (runs of consecutive noise steps, episodes that end on one), and the environment's default 5 %
-        "noise_all": _two_agent_cfg(33, dict(min_memory=33, capacity=500), dict(min_memory=20, capacity=500), env=dict(noise_prob=1.0)),
-        "noise_most": _two_agent_cfg(100, dict(min_memory=50, capacity=53), dict(min_memory=10, capacity=53), env=dict(noise_prob=0.6)),
-        "noise_rare": _two_agent_cfg(100, dict(), dict(actions=9, states=37), env=dict(noise_prob=0.05)),
-    }[case]
+    cfg = TWO_AGENT_CASES[case]
     for dtype, seed in ((np.float32, 41), (np.float64, 42)):
-        _philox_case(cfg, 40, 4, dtype, seed=seed, run_id0=3, hp=(case in ("partial_chunks", "noise_most")),
-                     chunks=[1, 3] if case in ("odd_T", "noise_all") else None)
+        _philox_case(cfg, 40, 4, dtype, seed=seed, run_id0=3, hp=(case in ("partial_chunks", "noise_most", "L17")),
+                     chunks=[1, 3] if case in ("odd_T", "noise_all", "T1", "L16") else None)
     if kernel_choice == "auto":
         assert _lib.last_kernel() == "lut2", _lib.last_kernel()
 
