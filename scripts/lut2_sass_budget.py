@@ -38,6 +38,10 @@ MARKERS = [
     ("run", "// ---- this warp's slot"),
     ("A", "// ---- A: draws"),
     ("B", "// ---- B: the episode"),
+    ("Bmap", "// ---- B.map"),
+    ("Bfill", "// ---- B.fill"),
+    ("Blog", "// ---- B.log"),
+    ("Bser", "} else if (!kNoise) {"),
     ("seq", "// states before every step"),
     ("trace", "// optional per-step traces"),
     ("C", "// ---- C: snapshot pass"),
@@ -50,12 +54,12 @@ MARKERS = [
     ("stats", "// epsilon decay"),
     ("run", "// ---- write the run back"),
 ]
-PHASES = ["A", "B", "seq", "C", "expand", "D", "E", "stats"]
+PHASES = ["A", "B", "Bmap", "Bfill", "Blog", "seq", "C", "expand", "D", "E", "stats"]
 
 
-def shape(dirty):
+def shape(dirty, events):
     T, L, chunk, NR, A = 100, 100, 16, 41, 21
-    return dict(T=T, L=L, chunk=chunk, chunks=math.ceil(L / chunk), NR=NR, A=A, dirty=dirty)
+    return dict(T=T, L=L, chunk=chunk, chunks=math.ceil(L / chunk), NR=NR, A=A, dirty=dirty, events=events)
 
 
 # loop trip counts per entry, by the text of the loop's `for` line (first match wins); the unroll factor of the source
@@ -66,7 +70,12 @@ def loop_trips(text, s):
     table = [
         (r"for \(int e = 0; e < E; \+\+e\)", None),                            # the epoch loop: counts are per epoch
         (r"for \(int t = lane; t < T; t \+= 32\)", math.ceil(T / 32)),          # A (and traces)
-        (r"for \(int n2 = T >> 1", T / 2 / 2),                                  # B, pairs, unroll 2
+        (r"for \(int n2 = T >> 1", T / 2 / 2),                                  # B step by step (Bser), pairs, unroll 2
+        (r"for \(int c0 = 0; c0 < T; c0 \+= 32\)", math.ceil(T / 32)),         # B.fill, 32 steps per pass
+        (r"for \(unsigned mw = m; mw != 0u", s["events"] / math.ceil(T / 32)),  # B.fill, the events of 32 steps
+        (r"for \(; t \+ 32 <= T; t \+= 32\)", T // 32),                        # B.log, 32 steps per iteration
+        (r"for \(; t \+ 8 <= T; t \+= 8\)", T % 32 // 8),                       # B.log, 8 steps
+        (r"for \(; t < T; \+\+t\)", T % 8),                                      # B.log, single steps
         (r"for \(int t = lane; t <= T; t \+= 32\)", math.ceil((T + 1) / 32)),   # seq
         (r"for \(int j = T - L1 \+ lane; j < T; j \+= 32\) reinterpret_cast", 0),  # C, unequal batches only (none at C2)
         (r"for \(int j = T - L0 \+ lane|for \(int j = T - L1 \+ lane", math.ceil(L / 32)),  # C, one agent per loop
@@ -166,6 +175,8 @@ def main():
     ap.add_argument("--src", default=None, help="thrl_scan_lut2.cuh the library was built from (default: next to --lib)")
     ap.add_argument("--build", action="store_true", help="build the library first (th_rl_b200.build)")
     ap.add_argument("--dirty", default="12,12", help="written compact rows per agent and epoch")
+    ap.add_argument("--events", type=float, default=8.0,
+                    help="exploration steps (events) per episode: the lane-parallel rollout's event loop trips")
     ap.add_argument("--loops", action="store_true", help="also list every loop with its static size and trip count")
     a = ap.parse_args()
     if a.build:
@@ -176,7 +187,7 @@ def main():
     with open(src) as f:
         src_lines = f.read().splitlines()
     phase = phase_of_lines(src_lines)
-    s = shape([int(x) for x in a.dirty.split(",")])
+    s = shape([int(x) for x in a.dirty.split(",")], a.events)
     instrs, labels = parse(disassemble(a.lib))
 
     # loops: backward branches (target index <= branch index), innermost first.  A loop's `for` is one of the `for` lines
@@ -231,8 +242,8 @@ def main():
             other[ph] = other.get(ph, 0.0) + n
     steps = 2 * s["T"]
     print("qtable_scan_lut2<float, true, false>  %s" % a.lib)
-    print("shape: T = L = %d, %d chunks, NR = %d, A = %d, written rows per epoch %s" %
-          (s["T"], s["chunks"], s["NR"], s["A"], "+".join(map(str, s["dirty"]))))
+    print("shape: T = L = %d, %d chunks, NR = %d, A = %d, written rows per epoch %s, events per episode %g" %
+          (s["T"], s["chunks"], s["NR"], s["A"], "+".join(map(str, s["dirty"])), s["events"]))
     print("%-8s %8s %14s" % ("phase", "static", "instr/ag-step"))
     for p in PHASES:
         print("%-8s %8d %14.2f" % (p, static[p], per_phase[p] / steps))

@@ -68,7 +68,11 @@ constexpr int kLut2MaxWarps = 24;  // float tables: 6 warps per scheduler at 80 
 template <typename QT> struct Lut2Warps { static constexpr int kMax = kLut2MaxWarps; };
 template <> struct Lut2Warps<double> { static constexpr int kMax = 16; };  // shared memory caps f64 tables at ~12 runs per SM: leave ptxas 128 registers
 constexpr int kLut2NoiseWarps = 16;  // noisy instantiation: every reachable row is staged (~16 KB per run), 13-14 runs fit: 128 registers
-constexpr int kLut2Chunk = 16;  // transitions expanded per pass of the update (16 lanes per agent)
+constexpr int kLut2Chunk = 16;
+// Episodes with at most this many exploration steps are played lane-parallel (phase B).  Each event costs one more lane-
+// parallel lift and replay of its 32 steps (~37 warp instructions); past ~12 events that costs more than the step-by-step
+// rollout (scripts/lut2_sass_budget.py --events).
+constexpr int kLut2MaxEvents = 12;  // transitions expanded per pass of the update (16 lanes per agent)
 
 // Row max / first argmax with the column count known to be <= 32 at compile time (kSmallA): one LDS per lane.
 template <typename QT, bool kSmallA>
@@ -336,7 +340,112 @@ __global__ void __launch_bounds__(kNoise ? 32 * kLut2NoiseWarps : 32 * Lut2Warps
           asm volatile("ld.shared.u16 %0, [%1];" : "=r"(s16) : "r"(next_a + 2u * joint));
           sig4 = s16;
         };
-        if (!kNoise) {
+        // Events: steps where an agent explores (keep != 0xffff).  Between events the greedy pairs GJ are frozen, so the next
+        // state is a fixed function of the current one, F(s) = nextS[joint(GJ[s])].  With few events the episode is played
+        // lane-parallel from the powers of F; otherwise (and past the limits of the lane-parallel plan) step by step.
+        unsigned evm0 = 0, evm1 = 0, evm2 = 0, evm3 = 0;  // event masks of steps 0-31, 32-63, 64-95, 96-127
+        bool par = false;
+        if (!kNoise && T > 0 && T <= 128 && NS < 64) {
+          const uint32_t* prew = reinterpret_cast<const uint32_t*>(pre);
+          auto evmask = [&](int t0) { const int t = t0 + lane; return __ballot_sync(kFull, t < T && prew[2 * t] != 0xffffu); };
+          evm0 = evmask(0); evm1 = evmask(32); evm2 = evmask(64); evm3 = evmask(96);
+          par = __popc(evm0) + __popc(evm1) + __popc(evm2) + __popc(evm3) <= kLut2MaxEvents;
+        }
+        if (!kNoise && par) {
+          // ---- B.map: successor powers.  Byte 0 of fp[k] in lane l is F^(2^k)(l), byte 1 is F^(2^k)(l + 32); states past NS
+          //      map to themselves.  The rollout goes 32 steps at a time, so five levels cover every distance.
+          uint32_t fp[5];
+          {
+            auto succ = [&](uint32_t s) -> uint32_t {
+              uint32_t n4 = 4u * s;
+              if (s <= (uint32_t)NS) {
+                uint32_t gj;
+                asm volatile("ld.shared.u32 %0, [%1];" : "=r"(gj) : "r"(gj_a + 4u * s));
+                asm volatile("ld.shared.u16 %0, [%1];" : "=r"(n4) : "r"(next_a + 2u * __dp4a(gj, dp_b, 0u)));
+              }
+              return n4 >> 2;
+            };
+            fp[0] = succ((uint32_t)lane) | (succ((uint32_t)lane + 32u) << 8);
+          }
+          // F^(2^k)(s) from level k's table: lane s & 31 holds it in byte s >> 5 (s < 64: one PRMT, selector 0x4440 + byte)
+          auto fwd = [&](uint32_t v, uint32_t s) -> uint32_t {
+            uint32_t r;
+            asm("prmt.b32 %0, %1, 0, %2;" : "=r"(r) : "r"(__shfl_sync(kFull, v, (int)s)), "r"((s >> 5) + 0x4440u));
+            return r;
+          };
+#pragma unroll
+          for (int k = 1; k < 5; ++k) fp[k] = fwd(fp[k - 1], fp[k - 1] & 0xffu) | (fwd(fp[k - 1], fp[k - 1] >> 8) << 8);
+          // F^d(s) for d < 32, d per lane
+          auto lift = [&](uint32_t s, uint32_t d) -> uint32_t {
+#pragma unroll
+            for (int k = 0; k < 5; ++k) {
+              const uint32_t n = fwd(fp[k], s);
+              s = (d >> k) & 1u ? n : s;
+            }
+            return s;
+          };
+
+          uint32_t sc = sig4_start >> 2;  // state before the first step of the 32
+          unsigned m = evm0;
+          for (int c0 = 0; c0 < T; c0 += 32) {
+            // ---- B.fill: lane = step t = c0 + lane.  Its state is F^(t - c0)(sc) up to the first event; each event, in
+            //      step order, restarts the lanes after it from the state it leads to.  Every step is played the same way,
+            //      events too: action pair = (greedy pair & keep) | forced, and the state it leads to (n4 = 4 x state)
+            const int t = c0 + lane;
+            uint32_t fx = 0xffffu, fy = 0u;
+            if (t < T) asm volatile("ld.shared.v2.u32 {%0, %1}, [%2];" : "=r"(fx), "=r"(fy) : "r"(pre_a + 8u * (uint32_t)t));
+            uint32_t st = lift(sc, (uint32_t)lane), kt, n4;
+            auto play = [&]() {
+              uint32_t gj;
+              asm volatile("ld.shared.u32 %0, [%1];" : "=r"(gj) : "r"(gj_a + 4u * st));
+              kt = (gj & fx) | fy;
+              asm volatile("ld.shared.u16 %0, [%1];" : "=r"(n4) : "r"(next_a + 2u * __dp4a(kt, dp_b, 0u)));
+            };
+            play();
+            for (unsigned mw = m; mw != 0u; mw &= mw - 1u) {
+              const int i = __ffs(mw) - 1;
+              const uint32_t nx = lift(__shfl_sync(kFull, n4, i) >> 2, (uint32_t)(lane - i - 1));
+              st = lane > i ? nx : st;
+              play();
+            }
+            if (t < T) asm volatile("st.shared.u16 [%0], %1;" ::"r"(rec_a + 2u * (uint32_t)t), "h"((uint16_t)kt) : "memory");
+            sc = __shfl_sync(kFull, n4, 31) >> 2;
+            m = c0 == 0 ? evm1 : c0 == 32 ? evm2 : evm3;
+          }
+          __syncwarp();
+          // ---- B.log: the four log sums in step order on lanes 0-3 (trainer.py:65-66), one DADD per step.  The lutLog
+          //      address of a step is one DP2A of its action pair: base + 32 A1 k0 + 32 k1
+          {
+            const uint32_t lq = log_a, wq = (32u * (uint32_t)A1) | (32u << 16);
+            auto add = [&](uint32_t a) {
+              asm volatile("ld.shared.f64 %0, [%1];" : "=d"(lg) : "r"(a));
+              acc = __dadd_rn(acc, lg);
+            };
+            auto eight = [&](int t) {  // eight steps per 16-byte load of rec
+              uint32_t r0, r1, r2, r3;
+              asm volatile("ld.shared.v4.u32 {%0, %1, %2, %3}, [%4];" : "=r"(r0), "=r"(r1), "=r"(r2), "=r"(r3) : "r"(rec_a + 2u * (uint32_t)t));
+              add(__dp2a_lo(wq, r0, lq)); add(__dp2a_hi(wq, r0, lq));
+              add(__dp2a_lo(wq, r1, lq)); add(__dp2a_hi(wq, r1, lq));
+              add(__dp2a_lo(wq, r2, lq)); add(__dp2a_hi(wq, r2, lq));
+              add(__dp2a_lo(wq, r3, lq)); add(__dp2a_hi(wq, r3, lq));
+            };
+            int t = 0;
+#pragma unroll 1
+            for (; t + 32 <= T; t += 32) { eight(t); eight(t + 8); eight(t + 16); eight(t + 24); }
+#pragma unroll 1
+            for (; t + 8 <= T; t += 8) eight(t);
+#pragma unroll 1
+            for (; t < T; ++t) {
+              uint32_t r0;
+              asm volatile("ld.shared.u16 %0, [%1];" : "=r"(r0) : "r"(rec_a + 2u * (uint32_t)t));
+              add(__dp2a_lo(wq, r0, lq));
+            }
+          }
+          uint32_t s16;
+          asm volatile("ld.shared.u16 %0, [%1];" : "=r"(kk) : "r"(rec_a + 2u * (uint32_t)(T - 1)));
+          asm volatile("ld.shared.u16 %0, [%1];" : "=r"(s16) : "r"(next_a + 2u * __dp4a(kk, dp_b, 0u)));
+          sig4 = s16;
+        } else if (!kNoise) {
         uint32_t pa = pre_a, ra = rec_a;
 #pragma unroll 2
         for (int n2 = T >> 1; n2 > 0; --n2, pa += 16u, ra += 4u) {  // two steps per 16-byte load of pre and per 4-byte store of rec
