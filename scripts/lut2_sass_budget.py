@@ -11,8 +11,8 @@ source (an instruction from a line of the kernel's prologue, a value re-derived 
   expand  D's per-chunk expansion + prologue   D       D's inner loop (one transition of each agent per iteration)
   E       greedy refresh, greedy-pair cache    stats   epsilon decay, logs, statistics
 Loops are the backward branches.  A loop's trip count per entry comes from the source line of its `for` (loop_trips below)
-at the C2 shape of bench.py: T = L = 100 steps, 16-transition chunks (7 per epoch), NR = 41 compact rows per agent, 21
-actions, and `--dirty` written compact rows per agent and epoch (scripts/lut2_chain_stats.py: ~26 distinct states per episode
+at the C2 shape of bench.py: T = L = 100 steps, 16-transition chunks (6 full ones through the unrolled body, 1 of 4
+through the loop), NR = 41 compact rows per agent, 21 actions, and `--dirty` written compact rows per agent and epoch (scripts/lut2_chain_stats.py: ~26 distinct states per episode
 at epsilon = 0.11, 12 at 0.026, 7.5 at 0.01).  Each instruction counts (executions per epoch of its innermost loop) / (2 T)
 warp instructions per agent-step; code outside the epoch loop (staging, write-back) is per run and is left out.
 
@@ -47,7 +47,9 @@ MARKERS = [
     ("C", "// ---- C: snapshot pass"),
     ("expand", "// chunk expansion, lane-parallel"),
     ("D", "// ---- D: the sequential pass"),
-    ("expand", "for (int c0 = 0; c0 < L0; c0 += kLut2Chunk)"),
+    ("expand", "for (; kSmallA && c0 + kLut2Chunk <= L0; c0 += kLut2Chunk) {"),
+    ("D", "const uint32_t cell_a = smem_base + cell_addr;"),
+    ("expand", "for (; c0 < L0; c0 += kLut2Chunk) {  // the partial last chunk"),
     ("D", "#pragma unroll 2\n          for (int j = n; j > 0; --j, --cd)"),
     ("Dsplit", "} else {\n        for (int ag = 0; ag < 2; ++ag)"),
     ("E", "// ---- E: refresh"),
@@ -80,8 +82,9 @@ def loop_trips(text, s):
         (r"for \(int j = T - L1 \+ lane; j < T; j \+= 32\) reinterpret_cast", 0),  # C, unequal batches only (none at C2)
         (r"for \(int j = T - L0 \+ lane|for \(int j = T - L1 \+ lane", math.ceil(L / 32)),  # C, one agent per loop
         (r"for \(int j = T - \(L0 > L1", math.ceil(L / 32)),                   # C, both agents per step
-        (r"for \(int c0 = 0; c0 < L0; c0 \+= kLut2Chunk\)", s["chunks"]),      # D chunks
-        (r"for \(int j = n; j > 0; --j, --cd\)", L / s["chunks"] / 2),          # D inner, unroll 2
+        (r"for \(; kSmallA && c0 \+ kLut2Chunk <= L0;", L // s["chunk"]),      # D full chunks (body unrolled)
+        (r"for \(; c0 < L0; c0 \+= kLut2Chunk\)", math.ceil(L % s["chunk"] / s["chunk"])),  # D, the partial last chunk
+        (r"for \(int j = n; j > 0; --j, --cd\)", L % s["chunk"] / 2),          # D, the partial chunk, unroll 2
         (r"for \(int c = 64 \+ lane", 0),                                     # E, rows from 64 on (none at C2)
         (r"for \(int i = lane; i < nd; i \+= 32\)", max(1, math.ceil(nd / 32))),  # E, lane per written row
         (r"for \(int k = 1; k < A; \+\+k\)", (A - 1) / 4),                     # E, row scan, unroll 4

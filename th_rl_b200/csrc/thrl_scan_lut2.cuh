@@ -90,6 +90,22 @@ __device__ __forceinline__ int lut2_row_argmax(const QT* row, int A, int lane, b
   const QT wm = warp_max(v);
   return (int)__reduce_min_sync(kFull, (in && v == wm) ? (unsigned)lane : 0xffffffffu);
 }
+// Row max with the lane's cell at shared-window address a (rows of <= 32 columns: one ld.shared per lane)
+__device__ __forceinline__ void lut2_lds(float& v, uint32_t a) { asm volatile("ld.shared.f32 %0, [%1];" : "=f"(v) : "r"(a)); }
+__device__ __forceinline__ void lut2_lds(double& v, uint32_t a) { asm volatile("ld.shared.f64 %0, [%1];" : "=d"(v) : "r"(a)); }
+template <typename QT>
+__device__ __forceinline__ QT lut2_row_max_at(uint32_t a) {
+  QT v;
+  lut2_lds(v, a);
+  return warp_max(v);
+}
+// Store v at shared-window address a on the lane whose li equals j: a predicated st.shared, no branch.
+__device__ __forceinline__ void lut2_sts_if(float v, uint32_t a, uint32_t li, uint32_t j) {
+  asm volatile("{ .reg .pred q; setp.eq.u32 q, %2, %3; @q st.shared.f32 [%0], %1; }" ::"r"(a), "f"(v), "r"(li), "r"(j) : "memory");
+}
+__device__ __forceinline__ void lut2_sts_if(double v, uint32_t a, uint32_t li, uint32_t j) {
+  asm volatile("{ .reg .pred q; setp.eq.u32 q, %2, %3; @q st.shared.f64 [%0], %1; }" ::"r"(a), "d"(v), "r"(li), "r"(j) : "memory");
+}
 
 // kNoise: demand noise (environments.py:28-31).  The intercept is redrawn in a few steps of an episode only, so the episode
 // is the noise-free rollout between those steps: a noise step computes its price, rewards and the four row encodes in f64 /
@@ -638,19 +654,60 @@ __global__ void __launch_bounds__(kNoise ? 32 * kLut2NoiseWarps : 32 * Lut2Warps
       if (L0 == L1) {
         // Both agents in one instruction stream, lanes 0-15 carrying agent 0 and lanes 16-31 agent 1.  Lane i of each half
         // expands transition c0+i of its agent and keeps the cell address, reward and (1-alpha)*old in registers; only the
-        // two next-row offsets of every transition go through shared memory (one uniform 8-byte load per iteration).  The
-        // row maxima are warp reductions, so every lane evaluates :72-74 and the lane that owns transition j stores.
+        // two next-row offsets of every transition go through shared memory (one uniform 8-byte load per transition, 16 bytes
+        // per two in a full chunk).  The row maxima are warp reductions, so every lane evaluates :72-74 and the lane that
+        // owns transition j stores.
         const int li = lane & (kLut2Chunk - 1);
         uint32_t rw_carry = kNoise ? 0u : rows_before(T - L0);
-        for (int c0 = 0; c0 < L0; c0 += kLut2Chunk) {
-          const int n = L0 - c0 < kLut2Chunk ? L0 - c0 : kLut2Chunk;
-          uint32_t row_off = 0, cell_addr = 0;
-          double2 v = make_double2(0.0, 0.0);
+        // shared-window addresses of this lane's column in each table and of the chunk, and the half, held in registers for
+        // the whole pass (not re-derived inside the unrolled chunk below)
+        uint32_t col0_a = smem_base + tab0_lane_off, col1_a = smem_base + tab1_lane_off, chunk_a = smem_base + chunk_off;
+        uint32_t hi_u = hi_half ? 1u : 0u;
+        asm volatile("" : "+r"(col0_a), "+r"(col1_a), "+r"(chunk_a), "+r"(hi_u));
+        // expansion of the chunk at c0 (n transitions): every lane's cell address and values, the next-row offsets of both
+        // agents to the chunk scratch
+        uint32_t cell_addr = 0;
+        double2 v = make_double2(0.0, 0.0);
+        auto stage = [&](int c0, int n) {
+          uint32_t row_off = 0;
           if (!kNoise) expand(min(c0 + li, L0 - 1), lane >> 4, L0, oma_h, rw_carry, row_off, cell_addr, v);
           else if (li < n) expand(c0 + li, lane >> 4, L0, oma_h, rw_carry, row_off, cell_addr, v);
           const uint32_t other = __shfl_xor_sync(kFull, row_off, 16);
           if (lane < n) *reinterpret_cast<uint2*>(smem + chunk_off + lane * 8) = make_uint2(row_off, other);
           __syncwarp();
+        };
+        int c0 = 0;
+        for (; kSmallA && c0 + kLut2Chunk <= L0; c0 += kLut2Chunk) {
+          // Full chunks, unrolled (rows of <= 32 columns: one load and one reduction per row): the offsets of two transitions
+          // per 16-byte load, read a pair ahead of the stores; no loop counter, and the store predicate is the lane against
+          // the (constant) transition index.  No branch between the expansion's shuffles and the end of the chunk, so the
+          // reductions need no divergence check.
+          stage(c0, kLut2Chunk);
+          const uint32_t cell_a = smem_base + cell_addr;
+          auto apply = [&](uint32_t ox, uint32_t oy, uint32_t j) {
+            const QT mx0 = lut2_row_max_at<QT>(col0_a + ox), mx1 = lut2_row_max_at<QT>(col1_a + oy);
+            const double mx = (double)(hi_u ? mx1 : mx0);
+            const double nv = __dadd_rn(v.y, __dmul_rn(alpha_h, __dadd_rn(v.x, __dmul_rn(gamma_h, mx))));  // :72-74
+            lut2_sts_if((QT)nv, cell_a, (uint32_t)li, j);                                                   // :75
+            __syncwarp();
+          };
+          uint32_t o[4];
+          asm volatile("ld.shared.v4.u32 {%0, %1, %2, %3}, [%4];" : "=r"(o[0]), "=r"(o[1]), "=r"(o[2]), "=r"(o[3]) : "r"(chunk_a));
+#pragma unroll
+          for (int j = 0; j < kLut2Chunk; j += 2) {
+            uint32_t on[4] = {0u, 0u, 0u, 0u};
+            if (j + 2 < kLut2Chunk)
+              asm volatile("ld.shared.v4.u32 {%0, %1, %2, %3}, [%4];" : "=r"(on[0]), "=r"(on[1]), "=r"(on[2]), "=r"(on[3])
+                           : "r"(chunk_a + 8u * (uint32_t)(j + 2)));
+            apply(o[0], o[1], (uint32_t)j);
+            apply(o[2], o[3], (uint32_t)j + 1u);
+#pragma unroll
+            for (int k = 0; k < 4; ++k) o[k] = on[k];
+          }
+        }
+        for (; c0 < L0; c0 += kLut2Chunk) {  // the partial last chunk (every chunk of rows wider than 32 columns)
+          const int n = L0 - c0 < kLut2Chunk ? L0 - c0 : kLut2Chunk;
+          stage(c0, n);
           uint32_t ca = smem_base + chunk_off;
           int cd = li;  // iterations until this lane's transition is applied
           uint32_t mx_, my_;  // next-row offsets, loaded one iteration ahead (off the store -> load chain; the slot after the
